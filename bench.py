@@ -3,6 +3,7 @@
 (depth-6, B=32) at 1/2/4/8 B200").
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload unet|cond|vae]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A step = one pass of the hot path over one batch: the stage-2 ("hr") U-Net forward on B=32 synthetic depth-6
@@ -24,6 +25,9 @@ Multi-GPU (BASELINE.json configs[2]): the B=32 shapes are SHARDED over the ranks
 no collective in the step loop (SURVEY.md 8e); one ragged all-gather of the final latents after the timed region.
 `--weak` keeps 32 shapes per GPU instead.  --workload cond = the class-conditional config (configs[4]);
 --workload vae = GraphVAE encode + decode at depth 8 (configs[3], HBM-bound regime).
+Weights, shapes and noise are seeded, so the same arguments give the same inputs on every run; --dump-outputs DIR
+writes what the last timed step returned (unet / cond: latent.npy = the updated latent, eps.npy = the U-Net output,
+all ranks' rows; vae: the decoder's logits and regression values per depth) as float32, at most 64 MB in all.
 """
 from __future__ import annotations
 import argparse
@@ -66,7 +70,14 @@ def parse():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-library-baseline', action='store_true')
     ap.add_argument('--no-roofline', action='store_true')
-    return ap.parse_args()
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write what the last timed step returned as DIR/<name>.npy (float32), to compare two builds')
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error('--steps must be >= 1 and --warmup >= 0')
+    if args.dump_outputs and args.impl != 'ours':
+        ap.error('--dump-outputs writes what --impl ours computed')
+    return args
 
 
 def config_for(args):
@@ -91,6 +102,24 @@ def randomise_(net, seed):
             fan = p[..., 0].numel() if p.dim() == 2 and p.shape[0] > p.shape[1] else p[0].numel()
             p.data.copy_(torch.randn(p.shape, generator=g) / max(fan, 1) ** 0.5)
     return net
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: each tensor as path/<name>.npy in float32.  Above DUMP_BYTES in all, every array keeps the same
+    share of its rows, chosen by a fixed seed (sorted), so that two builds with the same arguments stay comparable."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    total = sum(t.numel() * 4 for t in arrays.values())
+    for name, t in arrays.items():
+        t = t.detach().float()
+        if total > DUMP_BYTES:
+            keep = max(1, int(t.shape[0] * DUMP_BYTES // total))
+            rows = torch.randperm(t.shape[0], generator=torch.Generator().manual_seed(0))[:keep].sort().values
+            t = t[rows.to(t.device)]
+        np.save(os.path.join(path, name + '.npy'), t.cpu().numpy())
 
 
 def _synth():
@@ -338,6 +367,7 @@ def run_ours(args):
         raise SystemExit('bench.py --impl ours needs a CUDA device: octfusion_b200 has no CPU path')
     torch.cuda.set_device(local)
     dev = torch.device('cuda', local)
+    torch.manual_seed(0)            # the nets' default init draws from the global generator: same weights every run
     if world > 1:
         dist.init_process_group('nccl', device_id=dev)
     if args.workload == 'vae':
@@ -418,6 +448,11 @@ def run_ours(args):
     # strong scaling: one step of the job = all ranks' shards done; weak: every rank does a full batch per step
     value = (world if args.weak else 1) * args.steps / (ms_total / 1000.0)
     kernels_per_step = int(st.kernels_per_step)
+    if args.dump_outputs:            # the last timed step's latent and U-Net output, all ranks' rows (the e2e legs reuse st)
+        out = {name: torch.cat(shard.all_gather_latents(t)) for name, t in (('latent', st.x), ('eps', st.eps))}
+        if rank == 0:
+            dump_outputs(args.dump_outputs, out)
+        del out
 
     # ---- e2e: public sampler API (HRStepper, CUDA-graph step), host buffers, H2D + D2H inside the timed region ----
     x_host = torch.randn((n6, cc)).pin_memory()
@@ -448,12 +483,11 @@ def run_ours(args):
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         return (world if args.weak else 1) * k / (float(ms.item()) / 1000.0)
-    k2 = max(3, args.steps)
-    e2e_serial_v = run_e2e(e2e_serial, max(3, min(args.steps, 10)))
-    e2e_v = run_e2e(e2e_piped, k2)
+    e2e_serial_v = run_e2e(e2e_serial, args.steps)
+    e2e_v = run_e2e(e2e_piped, args.steps)
     e2e = {'value': e2e_v, 'unit': UNIT,
            'h2d_bytes_per_step': n6 * cc * 4 + 8, 'd2h_bytes_per_step': n6 * cc * 4,
-           'steps': k2, 'serial_value': e2e_serial_v,
+           'steps': args.steps, 'serial_value': e2e_serial_v,
            'path': 'sampler.HRStepper.step_host(pinned host latent, ..., pinned host result), per rank: H2D + [CUDA-graph replay of '
                    'U-Net forward + DDIM update] + D2H every step; double-buffered, the copies of step i run on copy streams '
                    'beside the compute of steps i-1 / i+1 (independent latents).  serial_value = the same with copy, step, '
@@ -576,10 +610,12 @@ def run_vae(args, dev, rank, world, real_stdout):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
     for _ in range(args.steps):
-        case['step']()
+        out = case['step']()
     e1.record()
     torch.cuda.synchronize()
     launches = _lib.launch_count() - c0
+    if args.dump_outputs and rank == 0:       # every rank decodes the same shapes
+        dump_outputs(args.dump_outputs, {'%s_d%d' % (k, d): t for k in ('logits', 'reg_voxs') for d, t in out[k].items()})
     ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)

@@ -2,7 +2,9 @@
 (CUDA) from the same synthetic split labels."""
 from __future__ import annotations
 import functools
+import hashlib
 import os
+import numpy as np
 import torch
 
 from octfusion_b200.synth import synth_splits
@@ -29,6 +31,26 @@ UNET_LABEL = [1, 3, 0, 4]
 def relerr(a, b):
     a, b = a.double().cpu(), b.double().cpu()
     return float((a - b).abs().max() / b.abs().max().clamp_min(1e-30))
+
+
+def digest(t) -> str:
+    """fingerprint for exact comparison with a stored reference tensor: dtype, shape and bytes (SHA-256), so that
+    large integer outputs (graphs, octree keys) are pinned bit for bit without storing them"""
+    a = np.ascontiguousarray(t.detach().cpu().numpy() if isinstance(t, torch.Tensor) else t)
+    h = hashlib.sha256(('%s %s ' % (a.dtype.str, a.shape)).encode())
+    h.update(a.tobytes())
+    return h.hexdigest()
+
+
+PIN_VALUES = 2048
+
+
+def pin_rows(t):
+    """every k-th row of `t` (rows = all but the last dimension), k chosen from t's shape so that about PIN_VALUES
+    values remain: the sample of a large reference output kept under golden/, and the same sample of the
+    output it is compared with"""
+    t = t.reshape(-1, t.shape[-1]) if t.dim() > 1 else t
+    return t[:: max(1, -(-t.numel() // PIN_VALUES))]
 
 
 @functools.lru_cache(maxsize=8)
